@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """bench.py — differentiable world-steps/s (fwd+bwd) of the batched Atlas timestep.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...         (one rank per GPU; batch shards, no data-path collective)
+
+--dump-outputs DIR writes what the last timed step returned to a caller of the headline path (next state, gradient w.r.t. the state,
+gradient w.r.t. the action; rank 0's shard) as DIR/<name>.npy, float32.  The inputs are seeded, so two builds can be compared output for
+output.  Above 64 MB in all, a fixed seeded sample of worlds (rows) is written instead.
 
 Headline workload (BASELINE.json configs[1]): Atlas humanoid (33 DoF, 28 moving bodies), contact-free, batch 4096 per GPU,
 one step = forward kernel + backward kernel over the whole batch, synthetic seeded inputs.
@@ -412,6 +416,21 @@ def rollout_leg(nb, torch, B, T, reps, dev, dist, rank, world_size):
                                    "tape_bytes_per_gpu": nb.rollout_tape_bytes(world, B, T, 8),
                                    "same_bits_as_full_tape": bool(torch.equal(gx0, gx0_k) and float(total) == float(total_k))}}
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> [B, k] host array, one row per world.  Writes DIR/<name>.npy (float32); above DUMP_BYTES in all, the same
+    seeded sample of rows from every array."""
+    B = next(iter(arrays.values())).shape[0]
+    per_world = sum(4 * a.shape[1] for a in arrays.values())
+    keep = min(B, (DUMP_BYTES - 4096) // per_world)
+    rows = np.arange(B) if keep == B else np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a[rows], dtype=np.float32))
+
+
 _REAL_STDOUT = None
 
 
@@ -440,7 +459,12 @@ def main():
     ap.add_argument("--precision", default="fp32", choices=["fp32", "fp64"])
     ap.add_argument("--lanes", type=int, default=0, help="threads cooperating on one world (0 = library picks from the batch size)")
     ap.add_argument("--no-extra", action="store_true", help="skip the cpu_baseline / e2e-independent extra contact legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step of the GPU headline path as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs covers the GPU headline path (--impl ours) only")
 
     rank = int(os.environ.get("RANK", "0"))
     world_size = int(os.environ.get("WORLD_SIZE", "1"))
@@ -592,6 +616,11 @@ def main():
     barrier()
     launches = _cabi.lib().nb2_launch_count() - l0
     total_ms = t0.elapsed_time(t1)
+    # the passes below reuse these buffers: keep the last timed step's outputs now
+    last = None
+    if args.dump_outputs:
+        d = sets[(args.warmup + args.steps - 1) % nsets]
+        last = {"next_state": d["nxt"].cpu().numpy(), "grad_state": d["gs"].cpu().numpy(), "grad_action": d["ga"].cpu().numpy()}
     # per-kernel times from a separate instrumented pass (an event after every launch), outside the timed region
     ne = min(args.steps, 50)
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(2 * ne + 1)]
@@ -731,6 +760,8 @@ def main():
         }
         if cpu_baseline is not None:
             out["cpu_baseline"] = cpu_baseline
+        if last is not None:
+            dump_outputs(args.dump_outputs, last)
         emit(out)
     if dist:
         dist.destroy_process_group()
